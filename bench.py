@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # own arm (B200 kernels)
     python bench.py --impl reference --gpus N --steps K ...   # CPU arm (compiled port of the path)
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's results as DIR/*.npy
 
 Workload ("step" = one batched solve of B instances per GPU, cold warm-start state, inputs resident
 in HBM): metric row of SURVEY.md §8d — Ackermann robot 4.6 x 1.6 m, horizon T=30, N=20 static
@@ -25,6 +26,26 @@ sys.path.insert(0, ROOT)
 T, N, E, R, ITERS = 30, 20, 4, 4, 50
 METRIC = 'MPC solves/sec (T=30, 20 obs, 50 ADMM iters)'
 WORKLOAD = 'metric row: acker, T=30, N=20 static polygons (E=4), 50 ADMM iterations, iter_threshold=0, cold start'
+DUMP_LIMIT = 64 << 20          # bytes of all files written by --dump-outputs
+
+
+def dump_outputs(out, path, seed=0):
+    """Write the result dict of one solve (u, s, resi_pri, resi_dual, status, iters) as <path>/<name>.npy: float fields as
+    float32, integer fields as float64 (exact).  A batch above DUMP_LIMIT is cut to a fixed, seeded sample of instances
+    whose indices are written as instance_index.npy, so that two builds run with the same arguments compare row for row.
+    u, s, status and iters repeat bitwise from run to run; resi_pri and resi_dual are float atomic sums over the cells and
+    differ in the last bits."""
+    arrs = {k: v.cpu().numpy() for k, v in out.items()}
+    arrs = {k: a.astype(np.float64 if a.dtype.kind in 'iu' else np.float32) for k, a in arrs.items()}
+    B = len(arrs['u'])
+    per_instance = sum(a[0].nbytes for a in arrs.values()) + 8
+    if B * per_instance > DUMP_LIMIT - 4096:            # 4 KB for the .npy headers
+        idx = np.sort(np.random.default_rng(seed).choice(B, (DUMP_LIMIT - 4096) // per_instance, replace=False))
+        arrs = {k: a[idx] for k, a in arrs.items()}
+        arrs['instance_index'] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(path, f'{k}.npy'), a)
 
 
 def algorithmic_bytes():
@@ -146,6 +167,8 @@ def run_config(args):
         out, gathered = step()
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -505,7 +528,13 @@ def main():
     ap.add_argument('--precision-sweep', action='store_true', help='--config B..E: float32 vs float64 su-QP by iteration')
     ap.add_argument('--su-fp32', action='store_true', help='float32 su-QP arithmetic (lower bound probe, not the metric)')
     ap.add_argument('--no-probes', action='store_true', help='skip early-stop / single-instance / closed-loop probes')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the results of the last timed step (rank 0\'s instances) as DIR/<name>.npy, at most 64 MB')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the results of the GPU path; the reference arm has none')
     if args.impl == 'reference':
         return run_reference(args)
     if args.config != 'metric':
@@ -564,6 +593,8 @@ def main():
         out = step(devin)
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)        # before the probes below reuse the solver's output buffers
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
